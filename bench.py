@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the hot path: FP64 CholInv (cholesky::cholinv::factor) on synthetic SPD input.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n SIZE]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n SIZE] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one cholinv::factor of the workload below on a resident (HBM) copy of the reference's own generator matrix
@@ -35,6 +35,20 @@ WORKLOADS = {  # n_gpus -> (n, c, bc_mult_dim)  ; base-case size b = 512 (N=1) /
 }
 STRONG_N = 32768
 STRONG_BCM = {1: -6, 2: -5, 4: -5, 8: -3}  # base case 512 global (1024 on the 2x2x2 grid, as in BASELINE config 3)
+DUMP_SAMPLES = 1 << 21  # per output, shared by all ranks: R and Rinv in FP64 come to 32 MB
+
+
+def sample_outputs(torch, np, pack, world, rank):
+    """--dump-outputs: the packed-upper R and Rinv that the last timed cholinv::factor returned, at positions drawn from a fixed seed
+    (all of them when an output is small), so that two builds can be compared entry for entry."""
+    out = {}
+    for name in ("R", "Rinv"):
+        t = getattr(pack, name)
+        k = min(t.numel(), DUMP_SAMPLES // world)
+        idx = np.sort(np.random.default_rng(rank).choice(t.numel(), k, replace=False))
+        key = name if world == 1 else f"{name}_rank{rank}"
+        out[key] = t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+    return out
 
 
 def clocks_sampler(stop: threading.Event, out: list, gpu_index: int):
@@ -310,6 +324,7 @@ def ours(args):
     stop.set()
     k_ms, k_flops, k_launches = ctx.profile_end()
     cnt = ctx.counters()
+    dumped = sample_outputs(torch, np, pack, world, rank) if args.dump_outputs else None  # before later steps reuse `pack`
     # The timed steps overlap kernels on two streams, which stretches event-bracketed launch durations.  The roofline
     # number is therefore taken from one extra step with the deferred stream disabled (same kernels, same launches).
     ctx.set_overlap(False)
@@ -529,6 +544,10 @@ def ours(args):
             else:
                 out["cpu_baseline"] = {"value": None, "unit": "TFLOP/s", "cores": os.cpu_count(), "kind": "reference", "sample": f"failed: {d}"}
         print(json.dumps(out))
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.barrier()
         cb.topo.release_contexts()
@@ -546,9 +565,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the N > 1 parity block")
     ap.add_argument("--no-extra", action="store_true", help="skip the strong-scaling and CholeskyQR2 records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of the last step's R and Rinv "
+                                                          "to DIR/<name>.npy (FP64, 32 MB)")
     args = ap.parse_args()
     if args.gpus not in WORKLOADS:
         raise SystemExit("--gpus must be one of 1, 2, 4, 8")
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        raise SystemExit("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     return reference_arm(args) if args.impl == "reference" else ours(args)

@@ -12,6 +12,7 @@ MKL's (blas/interface.hpp:43-97, lapack/interface.hpp:30-58).
 """
 from __future__ import annotations
 
+import json
 import math
 import numpy as np
 import scipy.linalg as sla
@@ -166,6 +167,16 @@ def unpack_upper(packed: np.ndarray, n: int) -> np.ndarray:
         out[: i + 1, i] = packed[off : off + i + 1]
         off += i + 1
     return out
+
+
+def load_dump(path: str):
+    """(meta, {name: array}) of a reference dump (tests/golden/*.npz).  Blocks that a rank holds identically to a lower rank
+    (replicas along z) are stored once; `same_as` names the stored copy of each omitted block."""
+    z = np.load(path)
+    arrs = {k: z[k] for k in z.files if k not in ("meta", "same_as")}
+    if "same_as" in z.files:
+        arrs.update({k: arrs[v] for k, v in json.loads(str(z["same_as"])).items()})
+    return json.loads(str(z["meta"])), arrs
 
 
 # --------------------------------------------------------------------------------------------------

@@ -34,6 +34,18 @@ def run(cmd, np_):
     out = subprocess.run(cmd, env=env, check=True, capture_output=True, text=True).stdout
     return json.loads(out.strip().splitlines()[-1])
 
+def save(name, meta, arrs):
+    """Replicas along z dump identical blocks: each distinct block is stored once and `same_as` maps the others to it (read back by
+    oracle.capital_oracle.load_dump), which keeps every fixture under 1 MB."""
+    kept, same_as = {}, {}
+    for k, a in arrs.items():
+        twin = next((j for j, b in kept.items() if np.array_equal(a, b)), None)
+        if twin is None:
+            kept[k] = a
+        else:
+            same_as[k] = twin
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), meta=json.dumps(meta), same_as=json.dumps(same_as), **kept)
+
 def main():
     only = set(sys.argv[1:])  # optional: regenerate the named fixtures only
     for name, P, n, ci, split, bcm, pol in CHOLINV:
@@ -45,7 +57,7 @@ def main():
             for r in range(P):
                 for k in ("A", "R", "Rinv"):
                     arrs[f"{k}_{r}"] = np.fromfile(os.path.join(td, f"d.{k}.{r}.bin"), dtype=np.float64)
-            np.savez_compressed(os.path.join(HERE, name + ".npz"), meta=json.dumps(meta), **arrs)
+            save(name, meta, arrs)
             print(name, meta)
     for name, P, var, m, n, c, ci, split, bcm in CACQR:
         if only and name not in only:
@@ -56,7 +68,7 @@ def main():
             for r in range(P):
                 for k in ("A", "Q", "R"):
                     arrs[f"{k}_{r}"] = np.fromfile(os.path.join(td, f"d.{k}.{r}.bin"), dtype=np.float64)
-            np.savez_compressed(os.path.join(HERE, name + ".npz"), meta=json.dumps(meta), **arrs)
+            save(name, meta, arrs)
             print(name, meta)
 
 if __name__ == "__main__":

@@ -3,7 +3,7 @@
 Checks the distributed CholInv (reference's 2x2x2 grid) and 1D CholeskyQR2 against the reference's own per-rank dumps
 (tests/golden/*_p8_*.npz), the oracle restatement, and the validators; rank 0 prints a summary line.
 """
-import json, os, sys
+import os, sys
 import numpy as np
 import torch
 import torch.distributed as dist
@@ -17,8 +17,7 @@ GOLD = os.path.join(ROOT, "tests", "golden")
 
 
 def load(name):
-    z = np.load(os.path.join(GOLD, name + ".npz"))
-    return json.loads(str(z["meta"])), z
+    return co.load_dump(os.path.join(GOLD, name + ".npz"))
 
 
 def main():

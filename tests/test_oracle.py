@@ -1,6 +1,6 @@
 """Pin the CPU restatement (oracle/capital_oracle.py) against the reference's own outputs
 (tests/golden/*.npz, dumped by the reference compiled in oracle/_ref) and against LAPACK."""
-import json, os
+import os
 import numpy as np
 import pytest
 import scipy.linalg as sla
@@ -10,8 +10,7 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def load(name):
-    z = np.load(os.path.join(GOLD, name + ".npz"))
-    return json.loads(str(z["meta"])), z
+    return co.load_dump(os.path.join(GOLD, name + ".npz"))
 
 
 def test_drand48_known_answers():
