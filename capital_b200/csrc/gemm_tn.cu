@@ -124,7 +124,9 @@ __global__ void __launch_bounds__(((BM / WM) * (BN / WN) + 4) * 32, MINB)
     const int t0 = min(nk, (int)blockIdx.z * per), t1 = min(nk, t0 + per);
     kb += t0 * BK;
     nk = t1 - t0;
-    if (nk == 0) return;
+    // An empty chunk has nothing to add to C (atomics), but the two-stage reduction reads every chunk's slice of kpart: it stores
+    // its zeros there, or the reduction would add whatever an earlier product left in the workspace.
+    if (nk == 0 && !p.kpart) return;
   }
   const int niter = nk * p.ncls;  // the k tiles of every operand class, one after the other
 
