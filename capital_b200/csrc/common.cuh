@@ -142,6 +142,15 @@ struct GemmOperands {
   const double* B[GEMM_NCLS_MAX] = {nullptr, nullptr};
   int64_t lda = 0, ldb = 0;
 };
+// Work enqueued on different streams of a context may run at the same time, so a workspace that a kernel reads after the host call
+// has returned is kept per stream (capital_ctx::stream_id; the distributed schedule numbers its streams the same way).
+static inline std::string stream_tag(const capital_ctx* ctx, cudaStream_t st) {
+  const int s = ctx->stream_id(st);
+  return s ? "_s" + std::to_string(s) : std::string();
+}
+// The scratch that gemm_tn copies an operand starting on an odd row into (operand 0 = A, 1 = B; operand class cls), on stream
+// `stream_id`.  The dry run of the distributed schedule records its uses under the same number.
+static inline int gemm_align_slot(int stream_id, int operand, int cls) { return (stream_id * 2 + operand) * GEMM_NCLS_MAX + cls; }
 capital_status_t gemm_tn_x(capital_ctx* ctx, cudaStream_t st, int64_t m, int64_t n, int64_t k, double alpha, const GemmOperands& ops,
                            double beta, double* C, int64_t ldc, int flags, int koff, int noff, const GemmXDev* x);
 capital_status_t gemm_tn(capital_ctx* ctx, cudaStream_t st, int64_t m, int64_t n, int64_t k, double alpha, const double* A,

@@ -189,6 +189,7 @@ struct Dist {
   size_t precv_stride[PEER_QC] = {};  // doubles per partial buffer of the class
   double* gath[2] = {nullptr, nullptr};
   int64_t gath_blk = 0;
+  int64_t bc_max = 0;  // widest base-case window of the recursion: what the gather buffers and the dense base-case block hold
   unsigned long long bc_count = 0;
   double *bcW = nullptr, *bcR = nullptr, *bcRi = nullptr, *bcRiT = nullptr;
   bool two_stream = true;
@@ -234,6 +235,16 @@ struct Dist {
   }
   void wr(int sid, int rank, const double* p, int64_t ldp, int64_t rows, int64_t cols, int64_t group = 0) {
     if (dry && p) rec(T_WRITE, sid, rank, (const char*)p - P->arena, ldp, rows, cols, group);
+  }
+  // dry runs only: the product of stream `sid` first copies each operand that starts on an odd row into the context's alignment
+  // scratch (gemm_tn.cu, launch), recorded as a write to scratch slot `gemm_align_slot` at the negative offset -1 - slot
+  void wr_align_scratch(int sid, const GemmOperands& ops, int64_t m, int64_t n, int64_t k) {
+    if (!dry) return;
+    for (int j = 0; j < ops.ncls; j++) {
+      const bool same = ops.A[j] == ops.B[j] && ops.lda == ops.ldb && m == n;  // B then reuses A's copy
+      if ((uintptr_t)ops.A[j] & 15) rec(T_WRITE, sid, me, -1 - gemm_align_slot(sid, 0, j), 0, k, m);
+      if (((uintptr_t)ops.B[j] & 15) && !same) rec(T_WRITE, sid, me, -1 - gemm_align_slot(sid, 1, j), 0, k, n);
+    }
   }
   capital_status_t wait_flags(int sid, const std::vector<Flag>& fl) {
     FlagList L_;
@@ -530,6 +541,7 @@ capital_status_t product_issue(Dist& D, int q, int64_t m, int64_t n, int64_t k, 
   if (D.xmode == 0) {
     if (D.dry) {
       for (int j = 0; j < D.nk; j++) { D.rd(sid, ops.A[j], ops.lda, k, m); D.rd(sid, ops.B[j], ops.ldb, k, n); }
+      D.wr_align_scratch(sid, ops, m, n, k);
       D.wr(sid, D.me, Cown, ldc, m, n);
       D.rec(T_PRODUCT, sid, q, 0, 0);
     } else if (trailing && trailing_uses_tf32(ctx, k * D.nk)) {
@@ -553,6 +565,7 @@ capital_status_t product_issue(Dist& D, int q, int64_t m, int64_t n, int64_t k, 
     CAP_TRY(D.wait_flags(sid, partner_flags(D, CTRL_DONE, q, 2 * seq - 1, false)));
     if (D.dry) {
       D.rd(sid, ops.A[0], ops.lda, k, m); D.rd(sid, ops.B[0], ops.ldb, k, n);
+      D.wr_align_scratch(sid, ops, m, n, k);
       const int64_t group = (int64_t)(seq * 8 + q + 1);
       D.wr(sid, D.me, Cown, ldc, m, n, group);
       for (int l = 0; l < D.c; l++)
@@ -590,6 +603,7 @@ capital_status_t product_issue(Dist& D, int q, int64_t m, int64_t n, int64_t k, 
   if (seq > (unsigned long long)nsets) CAP_TRY(D.wait_flags(sid, partner_flags(D, CTRL_RED, q, seq - nsets, false)));
   if (D.dry) {
     for (int j = 0; j < D.nk; j++) { D.rd(sid, ops.A[j], ops.lda, k, m); D.rd(sid, ops.B[j], ops.ldb, k, n); }
+    D.wr_align_scratch(sid, ops, m, n, k);
     D.wr(sid, D.me, own_set, ldp, m, n);
     for (int l = 0; l < D.c; l++)
       if (l != D.g.z) D.wr(sid, rank_of(D.g, D.g.x, D.g.y, l), recv_set + (size_t)(D.g.z < l ? D.g.z : D.g.z - 1) * stride, ldp, m, n);
@@ -694,6 +708,10 @@ capital_status_t base_case(Dist& D, int64_t o, int64_t s, int pending) {
   capital_ctx* ctx = D.ctx;
   const capital_grid_t& g = D.g;
   const int d = D.d;
+  if (s > D.bc_max) {  // dry runs too: a trace that passes here cannot write past a gather buffer into a peer's arena
+    ctx->set_error("distributed base case: window of " + std::to_string(s) + " exceeds the reserved " + std::to_string(D.bc_max));
+    return CAPITAL_ERR_UNSUPPORTED;
+  }
   CAP_TRY(need_cols(D, S_CHAIN, o + s));
   CAP_TRY(D.ev_wait(S_CHAIN, pending));
   double* Wo = D.W.own + o * D.ld + o;
@@ -768,6 +786,22 @@ capital_status_t dist_left_done(Dist& D, int64_t col_end, int depth) {
 inline bool node_splits(const Dist& D, int64_t s) {
   const int64_t s1 = s >> D.split;
   return !(s <= D.bc_local || s1 < D.split || s1 == 0);
+}
+// widest base-case window below a node of local size s.  Not bounded by bc_local alone: with split > 1 a node also stops when
+// s >> split < split (up to 7 wide for split = 2, 23 for split = 3).
+int64_t max_base_window(const Dist& D, int64_t s) {
+  if (!node_splits(D, s)) return s;
+  const int64_t s1 = s >> D.split;
+  return std::max(max_base_window(D, s1), max_base_window(D, s - s1));
+}
+// the two gather buffers of the base case (d > 1): d^2 slots of the widest window each
+void layout_gather(Layout& lay, Dist& D) {
+  D.bc_max = max_base_window(D, D.L);
+  D.gath_blk = 0;
+  if (D.d > 1) {
+    D.gath_blk = packed_ld(D.bc_max) * D.bc_max;
+    for (int i = 0; i < 2; i++) D.gath[i] = lay.take((size_t)D.gath_blk * D.d * D.d);
+  }
 }
 
 // cholinv::invoke (cholinv.hpp:87-165) on the local window [o, o+s).  `pending`: event after which the part of the window outside
@@ -892,12 +926,7 @@ size_t cholinv_layout(Dist& D, char* base) {
     layout_exchange(lay, D, q, mx, mx);
     if (q >= Q_FAR0) sz = sz - s1q;  // the right child is the larger one
   }
-  D.gath_blk = 0;
-  if (D.d > 1) {
-    const int64_t s = std::max<int64_t>(D.bc_local, 1) * 2;  // base-case windows are <= 2 bc_local - 1 (a node splits above bc_local)
-    D.gath_blk = packed_ld(s) * s;
-    for (int i = 0; i < 2; i++) D.gath[i] = lay.take((size_t)D.gath_blk * D.d * D.d);
-  }
+  layout_gather(lay, D);
   return lay.off;
 }
 
@@ -999,7 +1028,7 @@ capital_status_t need_comm(capital_ctx* ctx) {
 capital_status_t bc_workspace(Dist& D) {
   capital_ctx* ctx = D.ctx;
   if (D.d == 1) return CAPITAL_OK;
-  const int64_t b = std::max<int64_t>(D.bc_local, 1) * 2 * D.d, ldb = round_up(b, 16);
+  const int64_t b = D.bc_max * D.d, ldb = round_up(b, 16);
   const size_t bytes = (size_t)ldb * b * 8;
   void* old = ctx->pool.count("bc_Ri") ? ctx->pool["bc_Ri"].p : nullptr;
   CAP_TRY(ctx->workspace("bc_W", bytes, (void**)&D.bcW));
@@ -1275,12 +1304,7 @@ size_t qr3_layout(Qr3& q, char* base) {
   layout_mat(lay, D, q.Rt, ld, nl, ROLE_X, false);
   layout_mat(lay, D, q.Rf, ld, nl, 0, false);
   layout_exchange(lay, D, Q_CHAIN, nl, std::max(ml, nl));
-  D.gath_blk = 0;
-  if (D.d > 1) {
-    const int64_t s = std::max<int64_t>(D.bc_local, 1) * 2;
-    D.gath_blk = packed_ld(s) * s;
-    for (int i = 0; i < 2; i++) D.gath[i] = lay.take((size_t)D.gath_blk * D.d * D.d);
-  }
+  layout_gather(lay, D);
   return lay.off;
 }
 capital_status_t qr3_setup(capital_ctx* ctx, Dist& D, Qr3& q, int64_t m, int64_t n, const capital_cholinv_args_t* ci_args, const char* tag) {
@@ -1305,7 +1329,7 @@ capital_status_t qr3_setup(capital_ctx* ctx, Dist& D, Qr3& q, int64_t m, int64_t
     qr3_layout(q, buf);
   } else {
     const size_t bytes = qr3_layout(q, nullptr);
-    CAP_TRY(arena_prepare(ctx, bytes, std::string(tag) + ":" + std::to_string(q.ml) + ":" + std::to_string(q.nl) + ":" + std::to_string(D.bc_local)));
+    CAP_TRY(arena_prepare(ctx, bytes, std::string(tag) + ":" + std::to_string(q.ml) + ":" + std::to_string(q.nl) + ":" + std::to_string(D.bc_local) + ":" + std::to_string(D.split)));
     qr3_layout(q, D.P->arena);
   }
   CAP_TRY(bc_workspace(D));

@@ -243,14 +243,6 @@ capital_status_t make_map_f32(capital_ctx* ctx, CUtensorMap* map, const float* b
   return CAPITAL_OK;
 }
 
-const char* stream_tag(const capital_ctx* ctx, cudaStream_t st) {
-  if (st == ctx->side) return "_s0";
-  if (st == ctx->side_deep[0]) return "_s1";
-  if (st == ctx->side_deep[1]) return "_s2";
-  if (st == ctx->hi) return "_hi";
-  return "";
-}
-
 }  // namespace
 
 capital_status_t gemm_tf32_init(capital_ctx* ctx) {

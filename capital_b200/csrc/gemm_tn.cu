@@ -288,8 +288,9 @@ capital_status_t launch(capital_ctx* ctx, cudaStream_t st, int64_t m, int64_t n,
   p.ncls = ops.ncls;
   // TMA fetches 16-byte granules: a window that starts on an odd row (8-byte aligned only) cannot be addressed by
   // box coordinates, so it is first copied to an aligned scratch (O(k m) bytes against O(k m n) flops; only odd
-  // split points of non-power-of-two sizes ever take this path).
-  const char* sfx = st == ctx->side ? "_side" : "";
+  // split points of non-power-of-two sizes ever take this path).  One scratch per stream: a product on another stream may still be
+  // reading its own copy.
+  const int sid = ctx->stream_id(st);
   int64_t la[GEMM_NCLS_MAX], lb[GEMM_NCLS_MAX];
   for (int c = 0; c < ops.ncls; c++) {
     la[c] = ops.lda; lb[c] = ops.ldb;
@@ -297,14 +298,14 @@ capital_status_t launch(capital_ctx* ctx, cudaStream_t st, int64_t m, int64_t n,
     const int64_t lds = round_up(k, 2);
     if ((uintptr_t)ops.A[c] & 15) {
       double* sc;
-      CAP_TRY(ctx->workspace(std::string("gemm_alignA") + sfx + std::to_string(c), (size_t)lds * m * 8, (void**)&sc));
+      CAP_TRY(ctx->workspace("gemm_align" + std::to_string(gemm_align_slot(sid, 0, c)), (size_t)lds * m * 8, (void**)&sc));
       CAP_TRY(copy_block(ctx, st, k, m, ops.A[c], ops.lda, sc, lds));
       if (same) { ops.B[c] = sc; lb[c] = lds; }
       ops.A[c] = sc; la[c] = lds;
     }
     if ((uintptr_t)ops.B[c] & 15) {
       double* sc;
-      CAP_TRY(ctx->workspace(std::string("gemm_alignB") + sfx + std::to_string(c), (size_t)lds * n * 8, (void**)&sc));
+      CAP_TRY(ctx->workspace("gemm_align" + std::to_string(gemm_align_slot(sid, 1, c)), (size_t)lds * n * 8, (void**)&sc));
       CAP_TRY(copy_block(ctx, st, k, n, ops.B[c], ops.ldb, sc, lds));
       ops.B[c] = sc; lb[c] = lds;
     }

@@ -48,19 +48,18 @@ def main():
             res = cb.cholinv.residual(A, args, topo)
             ok &= er < 1e-13 and ei < 1e-13 and same_zeros and res < 1e-14
             msgs.append(f"{name}: dR={er:.1e} dRinv={ei:.1e} zeros={same_zeros} res={res:.1e}")
-        # --- split = 2 (left child = a quarter, cholinv.hpp:92,107): reference dump.  REPORTED, NOT GATING: the parameter's first run on
-        # the GPU path is whoever executes this (the schedule itself is replayed on CPU, tests/test_dist_protocol.py) ---
-        try:
-            meta, z = load("cholinv_p8_n256_ci1_split2")
-            n = meta["n"]
-            A = cb.matrix(n, n, 2, 2).distribute_symmetric(topo)
-            args = cb.cholinv.info(meta["complete_inv"], meta["split"], meta["bc_mult_dim"], "U")
-            cb.cholinv.factor(A, args, topo)
-            er = np.abs(args.R.cpu().numpy() - z[f"R_{rank}"]).max() / np.abs(z[f"R_{rank}"]).max()
-            ei = np.abs(args.Rinv.cpu().numpy() - z[f"Rinv_{rank}"]).max() / np.abs(z[f"Rinv_{rank}"]).max()
-            msgs.append(f"cholinv_p8_n256_ci1_split2 (not gating): dR={er:.1e} dRinv={ei:.1e} res={cb.cholinv.residual(A, args, topo):.1e}")
-        except Exception as ex:  # noqa
-            msgs.append("cholinv_p8_n256_ci1_split2 (not gating): " + repr(ex)[:120])
+        # --- split = 2 (left child = a quarter, cholinv.hpp:92,107): reference dump ---
+        meta, z = load("cholinv_p8_n256_ci1_split2")
+        n = meta["n"]
+        A = cb.matrix(n, n, 2, 2).distribute_symmetric(topo)
+        args = cb.cholinv.info(meta["complete_inv"], meta["split"], meta["bc_mult_dim"], "U")
+        cb.cholinv.factor(A, args, topo)
+        er = np.abs(args.R.cpu().numpy() - z[f"R_{rank}"]).max() / np.abs(z[f"R_{rank}"]).max()
+        ei = np.abs(args.Rinv.cpu().numpy() - z[f"Rinv_{rank}"]).max() / np.abs(z[f"Rinv_{rank}"]).max()
+        same_zeros = np.array_equal(args.Rinv.cpu().numpy() == 0, z[f"Rinv_{rank}"] == 0)
+        res = cb.cholinv.residual(A, args, topo)
+        ok &= er < 1e-13 and ei < 1e-13 and same_zeros and res < 1e-14
+        msgs.append(f"cholinv_p8_n256_ci1_split2: dR={er:.1e} dRinv={ei:.1e} zeros={same_zeros} res={res:.1e}")
         # --- oracle restatement at a size with several distributed levels + ragged local sizes ---
         for n, ci, bcm in (((768, 1, -2), (1536, 0, -3)) if small else ((1024, 1, -2), (1536, 0, -3), (4096, 0, -3))):
             A = cb.matrix(n, n, 2, 2).distribute_symmetric(topo)

@@ -7,14 +7,16 @@ it; a flag wait stalls the stream until the flag reaches the value) and checked 
   * deadlock freedom: the replay must drain every stream of every rank;
   * data races: two accesses to overlapping windows of the same rank's arena, at least one a write, must be ordered by
     happens-before (vector clocks) -- i.e. every operand a product reads from a mirror slot was pushed AND waited for, and
-    nothing of the next factorization overwrites what the previous one may still be reading.
+    nothing of the next factorization overwrites what the previous one may still be reading;
+  * scratch conflicts: a product whose operand starts on an odd row first copies it into an alignment scratch of its stream
+    (gemm_tn.cu); two uses of one scratch must be ordered too.
 """
 import ctypes as C
-import itertools
 import numpy as np
 import pytest
 import capital_b200 as cb
 from capital_b200 import _lib
+import dist_cases
 
 T_WAIT, T_SIGNAL, T_PRODUCT, T_EVREC, T_EVWAIT, T_DMA, T_KERNEL, T_READ, T_WRITE, T_MAT = range(1, 11)
 NSTREAM = 12
@@ -39,12 +41,15 @@ class Replay:
         self.nclk = self.P * NSTREAM
         self.streams = [[[] for _ in range(NSTREAM)] for _ in range(self.P)]
         self.mats = [[] for _ in range(self.P)]
+        self.recorded = [set() for _ in range(self.P)]  # events each rank records somewhere in its trace
         for r, tr in enumerate(traces):
             for rec in tr:
                 if rec[0] == T_MAT:
                     self.mats[r].append((int(rec[2]), int(rec[3]), int(rec[4])))
                 else:
                     self.streams[r][int(rec[1])].append(tuple(int(v) for v in rec))
+                    if rec[0] == T_EVREC:
+                        self.recorded[r].add(int(rec[2]))
         self.head = [[0] * NSTREAM for _ in range(self.P)]
         self.clock = [[np.zeros(self.nclk, dtype=np.int64) for _ in range(NSTREAM)] for _ in range(self.P)]
         self.flags = {}      # (rank, word) -> (value, clock)
@@ -91,8 +96,7 @@ class Replay:
             e = self.events.get((r, op[2]))
             if e is None:
                 # CUDA: waiting for an event that was never recorded is a no-op -- but the schedule never does that on purpose
-                own = [o for st in self.streams[r] for o in st if o[0] == T_EVREC and o[2] == op[2]]
-                assert own, f"rank {r}: wait for event {op[2]} that is never recorded"
+                assert op[2] in self.recorded[r], f"rank {r}: wait for event {op[2]} that is never recorded"
                 return False
             self.clock[r][s] = np.maximum(clk, e)
             self.tick(r, s)
@@ -136,14 +140,16 @@ class Replay:
         return None
 
     def races(self):
+        """Unordered conflicting pairs: (key, rect, R/W, (rank, stream), rect, R/W, (rank, stream)).  key[1] == "scratch" marks a
+        conflict on a GEMM's operand-alignment scratch (a buffer of the rank's context, outside the arena) rather than in the arena."""
         buckets = {}
         for a in self.accesses:
             rank, off, ld, rows, cols = a[:5]
-            sl = self.slot_of(rank, off)
-            if sl is None or sl[1] != ld:
-                key, r0, c0 = (rank, off, "raw"), 0, 0   # 1-D buffers (gather slots): whole-buffer granularity per base address
+            if off < 0:  # scratch slot -off - 1 of the rank's context: every use overlaps every other
+                key, rect = (rank, "scratch", -off - 1), (0, 1, 0, 1)
+            elif (sl := self.slot_of(rank, off)) is None or sl[1] != ld:
+                key = (rank, "raw")   # 1-D buffers (gather slots): byte ranges
                 rect = (off, off + rows * cols * 8, 0, 1)
-                key = (rank, "raw")
             else:
                 e = (off - sl[0]) // 8
                 c0, r0 = divmod(e, ld)
@@ -152,19 +158,25 @@ class Replay:
             buckets.setdefault(key, []).append((rect, a))
         bad = []
         for key, lst in buckets.items():
-            for (ra, a), (rb, b) in itertools.combinations(lst, 2):
-                if not (a[5] or b[5]):
-                    continue
-                if a[5] and b[5] and a[6] and a[6] == b[6]:
-                    continue  # cooperating writers of one fused product (disjoint tiles)
-                if ra[0] >= rb[1] or rb[0] >= ra[1] or ra[2] >= rb[3] or rb[2] >= ra[3]:
-                    continue
-                wa, wb = a[8], b[8]
-                ia, ib = wa[0] * NSTREAM + wa[1], wb[0] * NSTREAM + wb[1]
-                a_before_b = a[9][ia] <= b[7][ia]   # a's end happens-before b's start
-                b_before_a = b[9][ib] <= a[7][ib]
-                if not (a_before_b or b_before_a):
-                    bad.append((key, ra, "W" if a[5] else "R", wa, rb, "W" if b[5] else "R", wb))
+            rect = np.array([r for r, _ in lst], dtype=np.int64).reshape(-1, 4)
+            wr = np.array([a[5] for _, a in lst], dtype=bool)
+            grp = np.array([a[6] for _, a in lst], dtype=np.int64)
+            who = np.array([a[8][0] * NSTREAM + a[8][1] for _, a in lst], dtype=np.int64)
+            start = np.array([a[7] for _, a in lst], dtype=np.int64).reshape(len(lst), -1)
+            end = np.array([a[9] for _, a in lst], dtype=np.int64).reshape(len(lst), -1)
+            end_own = end[np.arange(len(lst)), who]
+            idx = np.arange(len(lst))
+            for i in np.nonzero(wr)[0]:  # every conflicting pair has a write: pair it with every later access and every earlier read
+                m = (idx > i) | ~wr
+                if grp[i]:
+                    m &= ~(wr & (grp == grp[i]))  # cooperating writers of one fused product (disjoint tiles)
+                m &= (rect[:, 0] < rect[i, 1]) & (rect[i, 0] < rect[:, 1]) & (rect[:, 2] < rect[i, 3]) & (rect[i, 2] < rect[:, 3])
+                m[i] = False
+                m &= end_own[i] > start[:, who[i]]     # not: the write's end happens-before the other's start
+                m &= end_own > start[i, who]           # not: the other's end happens-before the write's start
+                for j in np.nonzero(m)[0]:
+                    (ra, a), (rb, b) = lst[min(i, j)], lst[max(i, j)]
+                    bad.append((key, ra, "W" if a[5] else "R", a[8], rb, "W" if b[5] else "R", b[8]))
         return bad
 
 
@@ -233,3 +245,67 @@ def test_single_stream_schedule_also_clean(monkeypatch):
     rp = Replay(traces)
     assert not rp.run((2, 2))
     assert not rp.races()
+
+
+def replay_case(case):
+    traces = [trace(case.size, r, case.c, case.n, case.ci, case.bcm, case.split) for r in range(case.size)]
+    rp = Replay(traces)
+    stuck = rp.run((case.c, case.d))
+    bad = rp.races()
+    arena = [b for b in bad if b[0][1] != "scratch"]
+    scratch = [b for b in bad if b[0][1] == "scratch"]
+    return rp, stuck, arena, scratch
+
+
+@pytest.mark.parametrize("case", dist_cases.all_cases(), ids=lambda c: f"p{c.size}-n{c.n}-ci{c.ci}-split{c.split}-{c.knobs}")
+def test_schedule_table_drains_without_races_or_scratch_conflicts(case, monkeypatch):
+    """Every configuration the GPU parity worker runs (tests/dist_cases.py).  Odd split points make every GEMM copy its misaligned
+    operands into its stream's alignment scratch first; the chain and the deferred streams of depths 1 and 2 run such products at
+    the same time, so one scratch shared between them is overwritten while another stream's GEMM still reads it."""
+    for v in dist_cases.KNOB_VARS:
+        monkeypatch.delenv(v, raising=False)
+    for k, v in dist_cases.KNOBS[case.knobs].items():
+        monkeypatch.setenv(k, v)
+    rp, stuck, arena, scratch = replay_case(case)
+    assert not stuck, f"deadlock: {len(stuck)} streams blocked, e.g. {stuck[:4]}"
+    assert not arena, f"{len(arena)} unordered conflicting arena accesses, e.g. {arena[:3]}"
+    assert not scratch, f"{len(scratch)} unordered uses of one alignment scratch, e.g. {scratch[:3]}"
+    if dist_cases.ragged(case):  # the pseudo-accesses of the scratch must be in the trace
+        assert sum(1 for a in rp.accesses if a[1] < 0) > 0
+
+
+def test_scratch_uses_of_different_streams_are_unordered():
+    """The scratch check has teeth: merged onto one scratch slot per rank (as when every stream shared one buffer), the uses of
+    the chain and of the deferred streams in a ragged row of the table are unordered."""
+    case = next(c for c in dist_cases.all_cases() if c.size == 8 and c.n == 2052 and c.split == 1 and c.knobs == "deferred")
+    with pytest.MonkeyPatch.context() as mp:
+        for k, v in dist_cases.KNOBS[case.knobs].items():
+            mp.setenv(k, v)
+        traces = [trace(case.size, r, case.c, case.n, case.ci, case.bcm, case.split) for r in range(case.size)]
+    merged = []
+    for tr in traces:
+        tr = tr.copy()
+        scr = (tr[:, 0] == T_WRITE) & (tr[:, 3] < 0)
+        assert scr.any()
+        tr[scr, 3] = -1
+        merged.append(tr)
+    rp = Replay(merged)
+    assert not rp.run((case.c, case.d))
+    bad = rp.races()
+    assert bad and all(b[0][1] == "scratch" for b in bad)
+    assert {b[3][1] for b in bad} | {b[6][1] for b in bad} >= {1, 3, 4}  # chain, deferred depth 1, deferred depth 2
+
+
+@pytest.mark.parametrize("size", sorted(dist_cases.GRIDS))
+@pytest.mark.parametrize("split", [1, 2, 3])
+@pytest.mark.parametrize("bcm", [0, -3, -5, -8])
+def test_base_case_windows_fit_their_buffers(size, split, bcm, monkeypatch):
+    """Local size 256: bc_mult_dim -8 leaves a local base case of 1, where a split = 2 (3) node still stops at up to 7 (23) rows.
+    base_case refuses any window wider than what the gather buffers and the dense block were sized for, in the dry run too, so a
+    trace with status 0 proves that every window of the recursion fits."""
+    for v in dist_cases.KNOB_VARS:
+        monkeypatch.delenv(v, raising=False)
+    c, d = dist_cases.GRIDS[size]
+    n = 256 * d
+    traces = [trace(size, r, c, n, 1, bcm, split) for r in range(size)]
+    assert not Replay(traces).run((c, d))

@@ -14,8 +14,7 @@
                     tools/tf32_emulate.py: 5e-9 / 1e-10), and > 1e-13 with the TF32 kernel's launch counter > 0 -- i.e. the
                     tensor-core path really ran.
 
-3. XPASS/XFAIL -- split = 2 of the FP64 path against the reference's dump and the oracle (a parameter added to the parity set after the
-   GPU budget was spent; its schedule is replayed on CPU, its oracle is pinned on CPU)."""
+3. GATING -- split = 2 of the FP64 path against the reference's dump and the oracle."""
 import json
 import os
 import subprocess
@@ -81,8 +80,7 @@ def test_cholinv_mixed_precision_trailing_update():
     assert d["R_rel_diff"]["tf32"] <= 1e-4 and d["R_rel_diff"]["tf32x3"] <= 1e-6
 
 
-# ---- not TF32: a parameter of the FP64 path whose first GPU run is this file too (kept here so that it cannot stop the suite early) ----
-@pytest.mark.xfail(strict=False, reason="split = 2 was added to the parity set after the round's GPU budget was spent: first GPU run (XPASS = parity holds)")
+# ---- not TF32: split = 2 of the FP64 path ----
 def test_cholinv_uneven_split_matches_reference_dump_and_oracle():
     """split = 2 (cholinv.hpp:92,107: the left child gets a quarter of the node): the reference's own dump, elementwise, and the numpy
     restatement (pinned to that dump on CPU) at a ragged size."""
